@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — headline benchmark of the B200-native LeetCUDA hot paths.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Primary line (BASELINE.json configs[1]): HGEMM fp16 M=N=K=8192 through the reference-facing op
 `hgemm_mma_m16n8k16_mma2x4_warp4x4x2_stages_dsmem_swizzle` (NN layout).  One "step" = one GEMM
@@ -30,6 +30,10 @@ single-GPU 16384^3 figure (`strong_scaling_n1`) the N > 1 values are to be compa
 
 --impl reference times the reference's CPU path (torch.matmul on the host cores, all threads) on
 the same workload as this arm at the same N; rank 0 only.
+
+--dump-outputs DIR (N = 1) writes, after the timed steps, what the last timed step of the HGEMM line and of
+each attention row returned to its caller: a fixed, seeded sample of rows as float32 DIR/<name>.npy (44 MB in
+all).  The inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -157,6 +161,15 @@ def settle(seconds: float = 0.75):
     time.sleep(seconds)
 
 
+def sample_rows(t, n: int, seed: int):
+    """A fixed, seeded sample of n rows of t (viewed as [rows, last dim]), as float32 on the host."""
+    import numpy as np
+    import torch
+    flat = t.reshape(-1, t.shape[-1])
+    idx = np.sort(np.random.default_rng(seed).choice(flat.shape[0], min(n, flat.shape[0]), replace=False))
+    return flat[torch.from_numpy(idx).to(t.device)].float().cpu().numpy()
+
+
 def cuda_time_ms(fn, steps, sync):
     import torch
     e0 = torch.cuda.Event(enable_timing=True)
@@ -255,8 +268,9 @@ def cpu_baselines():
 
 
 def attention_row(torch, dev, world, rank, args, sync, shape, op, op_name, metric, kernel, peak_tf, peak_src, traffic_file,
-                  host_op, want_e2e):
-    """One attention config: device-timed value, roofline, vendor SDPA, e2e through the host-buffer entry."""
+                  host_op, want_e2e, dumps=None, dump_name=None):
+    """One attention config: device-timed value, roofline, vendor SDPA, e2e through the host-buffer entry.
+    With `dumps`, a row sample of the output of the last timed step goes to dumps[dump_name]."""
     import torch.distributed as dist
     import torch.nn.functional as F
     from leetcuda_b200 import _capi
@@ -280,6 +294,8 @@ def attention_row(torch, dev, world, rank, args, sync, shape, op, op_name, metri
     with ClockSampler(dev.index) as row_clk:
         fms = cuda_time_ms(fstep, args.steps, sync)
     launches = _capi.launch_count() - l1
+    if dumps is not None:
+        dumps[dump_name] = sample_rows(outs[(args.steps - 1) % nsets], (1 << 20) // D, seed=D)   # 4 MB
     tf = torch.tensor([fms], device=dev, dtype=torch.float64)
     if world > 1:
         dist.all_reduce(tf, op=dist.ReduceOp.MAX)
@@ -337,8 +353,12 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-secondary", action="store_true", help="skip the attention metrics and the next rows")
     ap.add_argument("--no-cpu", action="store_true", help="skip the CPU baseline leg")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write a fixed row sample of what the last timed step of each GPU row computed to DIR/<name>.npy")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3)
+    if args.impl == "reference" and args.dump_outputs:
+        ap.error("--dump-outputs writes the GPU rows' outputs; --impl reference has none")
 
     if args.impl == "reference":
         run_reference(args)
@@ -353,7 +373,10 @@ def main():
     torch.cuda.set_device(local)
     dev = torch.device("cuda", local)
     if world > 1:
+        if args.dump_outputs:
+            raise SystemExit("--dump-outputs runs on one GPU")
         dist.init_process_group("nccl", device_id=dev)
+    dumps = {} if args.dump_outputs else None
 
     from leetcuda_b200 import _capi, ffpa_attn, flash_attn, hgemm
     from leetcuda_b200 import dist as bdist
@@ -420,6 +443,8 @@ def main():
     with ClockSampler(local) as clk:
         ms = cuda_time_ms(step, args.steps, sync)
     launches = _capi.launch_count() - l0
+    if dumps is not None:   # before the roofline and cuBLAS legs below write into Cs again
+        dumps["hgemm_c"] = sample_rows(Cs[(args.steps - 1) % NSETS], 1024, seed=0)   # 32 MB
     t = torch.tensor([ms], device=dev, dtype=torch.float64)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -487,14 +512,14 @@ def main():
             torch, dev, world, rank, args, sync, FA, flash_attn.flash_attn_mma_stages_split_q_shared_qkv,
             "flash_attn_mma_stages_split_q_shared_qkv", "FA-2 fp16 TFLOPS @B4H32N4096D128 (matmul FLOPs 4BHN^2D)",
             "attn_fwd_kernel<128> (two query tiles per CTA)", peak_tf, peak_src, "attn_traffic.json",
-            flash_attn.fmha_host, True)
+            flash_attn.fmha_host, True, dumps, "attn_o_d128")
         launches += nl
         try:
             config4, nl = attention_row(
                 torch, dev, world, rank, args, sync, FF, ffpa_attn.ffpa_mma_acc_f32_L1,
                 "ffpa_mma_acc_f32_L1", "FFPA fp16 TFLOPS @B2H16N2048D512 (matmul FLOPs 4BHN^2D)",
                 "attn_pair_fwd_kernel (one query tile per CTA pair, cta_group::2)", peak_tf, peak_src,
-                "attn_pair_traffic.json", flash_attn.fmha_host, True)
+                "attn_pair_traffic.json", flash_attn.fmha_host, True, dumps, "ffpa_o_d512")
             launches += nl
         except Exception as e:
             config4 = {"error": f"{type(e).__name__}: {e}"}
@@ -504,7 +529,7 @@ def main():
                 torch, dev, world, rank, args, sync, (FA[0], FA[1], FA[2], 64), flash_attn.flash_attn_mma_stages_split_q_shared_qkv,
                 "flash_attn_mma_stages_split_q_shared_qkv", "FA-2 fp16 TFLOPS @B4H32N4096D64 (matmul FLOPs 4BHN^2D)",
                 "attn_fwd_kernel<64> (two query tiles per CTA, persistent grid)", peak_tf, peak_src, "attn_d64_traffic.json",
-                flash_attn.fmha_host, False)
+                flash_attn.fmha_host, False, dumps, "attn_o_d64")
             launches += nl
         except Exception as e:
             attn_d64 = {"error": f"{type(e).__name__}: {e}"}
@@ -604,6 +629,12 @@ def main():
                              "total work fixed); strong_scaling_n1 on the N=1 line is the one-GPU 16384^3 figure"),
         }
         print(json.dumps(line), flush=True)
+    if dumps is not None:
+        import numpy as np
+        out = Path(args.dump_outputs)
+        out.mkdir(parents=True, exist_ok=True)
+        for name, arr in dumps.items():
+            np.save(out / f"{name}.npy", arr)
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()

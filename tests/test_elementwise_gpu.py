@@ -130,6 +130,7 @@ def test_rope_qk_and_attention(shape):
 # against the recorded outputs of the reference's own kernels (oracle/_ref rebuilt for sm_100a with the reference's
 # flags, --use_fast_math included; oracle/gen_golden.py on a B200)
 # ---------------------------------------------------------------------------------------------------------------
+import json  # noqa: E402
 from pathlib import Path  # noqa: E402
 
 from oracle.gen_golden import RMSNORM_CASES, ROPE_CASES, rowwise_inputs  # noqa: E402
@@ -169,6 +170,7 @@ def test_rms_norm_vs_reference_golden(case):
         pytest.skip("golden file not generated yet")
     g = np.load(f)
     gain = 1.25
+    sub = json.loads(str(g["meta"]))["subsample"]          # the goldens keep every sub-th row
     x32 = torch.from_numpy(rowwise_inputs(R, K, seed)).cuda()
     x16 = x32.half()
     y32, y16 = torch.empty_like(x32), torch.empty_like(x16)
@@ -176,8 +178,8 @@ def test_rms_norm_vs_reference_golden(case):
     rms_norm.rms_norm_f16x8_pack_f32(x16, y16, gain)
     torch.cuda.synchronize()
     for name in ("rms_norm_f32", "rms_norm_f32x4"):
-        np.testing.assert_allclose(y32.cpu().numpy()[::4], g[name], rtol=1e-5, atol=1e-6, err_msg=name)
-    got16 = y16.cpu().numpy().astype(np.float32)[::4]      # the goldens keep every 4th row
+        np.testing.assert_allclose(y32.cpu().numpy()[::sub], g[name], rtol=1e-5, atol=1e-6, err_msg=name)
+    got16 = y16.cpu().numpy().astype(np.float32)[::sub]
     for name in ("rms_norm_f16x8_f32", "rms_norm_f16x8_pack_f32", "rms_norm_f16_f32"):      # fp32 statistics: one fp16 ulp
         np.testing.assert_allclose(got16, g[name].astype(np.float32), rtol=1e-3, atol=1e-3, err_msg=name)
     for name in ("rms_norm_f16_f16", "rms_norm_f16x2_f16", "rms_norm_f16x8_f16", "rms_norm_f16x8_pack_f16"):
