@@ -105,7 +105,8 @@ int b200_hgemm_f16_rows_fused(const void* a_shard, const void* b, void* c_full, 
                               int b_layout, int row0, void* stream);
 
 /* O = softmax(Q K^T * scale) V per (batch, head); fp16 in/out, fp32 softmax
- * statistics and fp32 accumulation; non-causal, no mask, no dropout.
+ * statistics and fp32 accumulation; non-causal, no mask, no dropout, equal query and key lengths
+ * (b200_fmha_fwd_f16_ex below adds the causal mask and separate lengths).
  *
  * Replaces every `void flash_attn_mma_stages_*(Q,K,V,O,int stages)` bound in
  * kernels/flash-attn/pybind/flash_attn.cc:168-224 (e.g. the shared-QKV launcher
@@ -139,6 +140,27 @@ int b200_fmha_fwd_f16(const void* q, const void* k, const void* v, void* o, int 
  * kernels/openai-triton/merge-attn-states/test_merge_attn_states.py:100-152). */
 int b200_fmha_fwd_f16_lse(const void* q, const void* k, const void* v, void* o, float* lse, int B,
                           int H, int N, int D, int v_transposed, float scale, void* stream);
+
+/* Attention with separate query / key lengths and an optional causal mask:
+ *   o[b,h,i] = sum_{allowed j} softmax_j(scale * q_i . k_j) v_j
+ * q, o: [B,H,Nq,D].  k: [B,H,Nk,D].  v: [B,H,Nk,D], or [B,H,D,Nk] with v_transposed.  lse: [B,H,Nq] fp32, may be
+ * NULL.  All of them fp16 (lse fp32), contiguous.
+ *   causal = 0: every query row attends to all Nk keys; any Nq, Nk >= 1.
+ *   causal = 1: query row i attends to the keys j <= i + (Nk - Nq): the BOTTOM-RIGHT alignment of FlashAttention-2
+ *               >= 2.1 (the last query row sees every key).  It equals the top-left alignment when Nq == Nk, and is
+ *               NOT what torch's scaled_dot_product_attention(is_causal=True) computes for Nq != Nk (top-left).
+ *               Requires Nk >= Nq, so that every row sees at least one key.
+ *   lse[b,h,i] = ln sum_{allowed j} exp(scale * q_i . k_j): the statistic of b200_fmha_fwd_f16_lse restricted to the
+ *   allowed keys, so two calls over disjoint key ranges can be combined with b200_merge_attn_states.
+ * B200_EINVAL for a null q/k/v/o, B, H, Nq, Nk or D <= 0, causal outside {0, 1}, causal with Nk < Nq, and
+ * v_transposed with Nk % 8 != 0; B200_ENOTSUP for the head dims b200_fmha_fwd_f16 rejects.  Numerics as
+ * b200_fmha_fwd_f16.  With causal = 0 and Nq == Nk the result is bit-identical to b200_fmha_fwd_f16{,_lse}.
+ * Kernels: those of b200_fmha_fwd_f16.  A causal work item (query tile) runs only the KV tiles up to its last
+ * row's diagonal and masks the keys past the diagonal, and the longest items are dispatched first.  The opt-in
+ * variants B200_ATTN_CG2=1, B200_ATTN_SPEC=2 and B200_ATTN_PAIR_PERSIST=1 are not taken when causal = 1 or
+ * Nq != Nk: the default kernel for the head dim runs instead. */
+int b200_fmha_fwd_f16_ex(const void* q, const void* k, const void* v, void* o, float* lse, int B, int H,
+                         int Nq, int Nk, int D, int v_transposed, int causal, float scale, void* stream);
 
 /* ------------------------------------------------------------------ SGEMM (TF32)
  * C[M,N] (fp32) = A[M,K] (fp32) x B on the tensor cores through tcgen05 kind::tf32 with fp32

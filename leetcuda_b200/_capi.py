@@ -39,6 +39,7 @@ SIGNATURES = {
     "b200_hgemm_f16_rows_fused": (_i, [_vp, _vp, _vp, _vp, ctypes.POINTER(ctypes.c_void_p), _i, _i, _i, _i, _i, _i, _vp]),
     "b200_fmha_fwd_f16": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _f, _vp]),
     "b200_fmha_fwd_f16_lse": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _f, _vp]),
+    "b200_fmha_fwd_f16_ex": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _f, _vp]),
     "b200_fmha_fwd_f16_rmsnorm": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _f, _f, _vp]),
     "b200_rope_f32": (_i, [_vp, _vp, _i, _i, _vp]),
     "b200_rope_qk_f16": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _i, _vp]),

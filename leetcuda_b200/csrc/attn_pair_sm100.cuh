@@ -65,16 +65,19 @@ constexpr int smem_bytes(int nq) {
 }
 
 struct Params {
-  int N;            // sequence length
-  int num_kv;       // ceil(N / BC)
+  int Nq;           // query rows (q, o, lse)
+  int Nk;           // keys (k, v)
+  int num_kv;       // ceil(Nk / BC)
+  int causal;       // 1: query row i sees the keys j <= i + Nk - Nq (bottom-right aligned; host guarantees Nk >= Nq;
+                    // one-shot launches only)
   int nq;           // D / 64: 64-wide d-chunks of Q / K (4, 6 or 8)
   int n_hi;         // D - 256: N of the second P.V instruction (0, 128 or 256)
   float scale_log2; // softmax scale * log2(e)
-  float* lse;       // optional [B*H, N] fp32: log-sum-exp of the scaled scores (natural log); nullptr = off
+  float* lse;       // optional [B*H, Nq] fp32: log-sum-exp of the scaled scores (natural log); nullptr = off
   float rms_g;      // > 0: fused RMS norm of the output rows over D (eps 1e-5), scaled by rms_g; see attn_sm100.cuh
   // persistent launches (kPersist): one cluster per SM pair walks the (batch*head, query tile) work items
   __half* o_ptr;    // O base pointer: the epilogue stores rows straight from registers (Q's smem is being reloaded)
-  int qtiles;       // ceil(N / 128): work items per (batch, head)
+  int qtiles;       // ceil(Nq / 128): work items per (batch, head)
   int total_items;  // qtiles * B * H
 };
 
@@ -119,10 +122,13 @@ attn_pair_fwd_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_co
   const int lane = threadIdx.x & 31;
   const uint32_t rank = cluster_ctarank();
   const bool leader = (rank == 0);
-  const int T = p.num_kv;
   // work items of this cluster; the KV tiles of all of them form one sequence g = it * T + j
   const int cid = static_cast<int>(blockIdx.x >> 1), ncl = static_cast<int>(gridDim.x >> 1);
   const int n_items = kPersist ? (p.total_items - cid + ncl - 1) / ncl : 1;
+  // causal (one-shot only): the clusters run their query tiles in reverse, heaviest first
+  const int qt0 = p.causal ? ncl - 1 - cid : cid;
+  // KV tiles per item: the two CTAs share every MMA, so the extent follows the last row of the cluster's 128-row tile
+  const int T = kPersist ? p.num_kv : attn_kv_tiles(p.causal, p.num_kv, p.Nq, p.Nk, qt0 * BR + BR, BC);
   const int total = n_items * T;
   auto item_coords = [&](int it, int& bh, int& q0) {     // q0: first query row of THIS CTA
     if constexpr (kPersist) {
@@ -131,7 +137,7 @@ attn_pair_fwd_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_co
       q0 = (w - bh * p.qtiles) * BR + static_cast<int>(rank) * ROWS;
     } else {
       bh = blockIdx.y;
-      q0 = cid * BR + static_cast<int>(rank) * ROWS;
+      q0 = qt0 * BR + static_cast<int>(rank) * ROWS;
     }
   };
   const int n_hi_cta = p.n_hi >> 1;           // d-columns of O_hi held by this CTA (64 or 128)
@@ -306,10 +312,17 @@ attn_pair_fwd_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_co
     float m_run = -INFINITY;
     float l_run = 0.f;                       // partial row sum over this thread's key halves
     uint8_t* p_gen = smem_gen + q_bytes;
+    int key_end = p.Nk;                      // one past the last key of this thread's row (keys past it: -inf)
 
     for (int g = 0; g < total; ++g) {
       const int it = g / T, j = g - it * T;
-      if (j == 0) { m_run = -INFINITY; l_run = 0.f; }      // a new work item
+      if (j == 0) {                                         // a new work item
+        m_run = -INFINITY;
+        l_run = 0.f;
+        int bh, q0;
+        item_coords(it, bh, q0);
+        key_end = attn_key_end(p.causal, p.Nq, p.Nk, q0 + row);
+      }
       const uint32_t tS = tmem_base + (g & 1) * 128 + lane_field;
       mbar_wait(s_full(g & 1), (g >> 1) & 1, 300 + (g & 1));
       tc_fence_after();
@@ -319,7 +332,7 @@ attn_pair_fwd_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_co
       tmem_ld_x32(tS + 64, sreg[2]);
       tmem_ld_x32(tS + 96, sreg[3]);
       tmem_ld_wait();
-      const int valid = p.N - j * BC - half * 128;    // keys of this thread's half that exist
+      const int valid = key_end - j * BC - half * 128;    // keys of this thread's half the row sees
       if (valid < 128) {
 #pragma unroll
         for (int cb = 0; cb < 4; ++cb)
@@ -423,8 +436,8 @@ attn_pair_fwd_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_co
       named_bar_sync(1, 128);
       const float l_row = l_run + xl[L ^ 64];
       float inv_l = 1.0f / l_row;
-      if (p.lse != nullptr && half == 0 && (q0 + row) < p.N)
-        p.lse[static_cast<size_t>(bh) * p.N + q0 + row] = 0.6931471805599453f * (m_run * c + log2f(l_row));
+      if (p.lse != nullptr && half == 0 && (q0 + row) < p.Nq)
+        p.lse[static_cast<size_t>(bh) * p.Nq + q0 + row] = 0.6931471805599453f * (m_run * c + log2f(l_row));
       if (p.rms_g > 0.f) {
         ss += xs[L ^ 64];
         inv_l *= rsqrtf(ss * inv_l * inv_l / static_cast<float>(NQ * 64) + 1e-5f) * p.rms_g;
@@ -451,8 +464,8 @@ attn_pair_fwd_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_co
           v[q4].w = pack_half2(__uint_as_float(o[q4 * 8 + 6]) * inv_l, __uint_as_float(o[q4 * 8 + 7]) * inv_l);
         }
         if constexpr (kPersist) {
-          if ((q0 + row) < p.N) {
-            __half* dst = p.o_ptr + (static_cast<size_t>(bh) * p.N + q0 + row) * (NQ * 64) + d0;
+          if ((q0 + row) < p.Nq) {
+            __half* dst = p.o_ptr + (static_cast<size_t>(bh) * p.Nq + q0 + row) * (NQ * 64) + d0;
 #pragma unroll
             for (int q4 = 0; q4 < 4; ++q4) *reinterpret_cast<uint4*>(dst + q4 * 8) = v[q4];
           }
@@ -472,7 +485,7 @@ attn_pair_fwd_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_co
       } else {
         fence_proxy_async_smem();
         named_bar_sync(1, 128);
-        if (warp == 0 && lane == 0 && q0 < p.N) {
+        if (warp == 0 && lane == 0 && q0 < p.Nq) {
           for (int b = 0; b < NQ; ++b)
             tma_store_3d(&tmap_o, smem_base + b * QBOX_BYTES, b * 64, q0, bh);
           tma_store_commit();

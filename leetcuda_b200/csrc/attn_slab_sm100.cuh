@@ -63,19 +63,22 @@ constexpr int smem_bytes(int nq_chunks) {
 }
 
 struct Params {
-  int N;            // sequence length
-  int num_kv;       // ceil(N / BC)
+  int Nq;           // query rows (q, o, lse)
+  int Nk;           // keys (k, v)
+  int num_kv;       // ceil(Nk / BC)
+  int causal;       // 1: query row i sees the keys j <= i + Nk - Nq (bottom-right aligned; host guarantees Nk >= Nq)
   int nq;           // DQ / 64: 64-wide d-chunks of Q/K
   int dv;           // output columns of this CTA's slab (multiple of 64, <= 256)
   int dsplit;       // slabs per query tile
   float scale_log2;
-  float* lse;       // optional [B*H, N] fp32 log-sum-exp output (written by slab 0), nullptr = off
+  float* lse;       // optional [B*H, Nq] fp32 log-sum-exp output (written by slab 0), nullptr = off
   float rms_g;      // > 0: fused RMS norm of the output rows (single-slab launches only, D <= 256); see attn_sm100.cuh
   int D;            // true head dim (mean of the RMS norm)
 };
 
 // kWide: Q resident, 32 KiB ring slots (K slot = two {64 d x 128 keys} boxes, V slot = 64 keys); else Q streamed, 16 KiB slots
-template <bool kWide>
+// kCausal: the causal mask (Params::causal), a separate instantiation so that the full-attention kernel is unchanged
+template <bool kWide, bool kCausal>
 __global__ void __launch_bounds__(kThreads, 1)
 attn_slab_fwd_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constant__ CUtensorMap tmap_k,
                    const __grid_constant__ CUtensorMap tmap_v, const __grid_constant__ CUtensorMap tmap_o,
@@ -107,11 +110,13 @@ attn_slab_fwd_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_co
   const int warp = __shfl_sync(0xffffffffu, threadIdx.x >> 5, 0);
   const int lane = threadIdx.x & 31;
   const int bh = blockIdx.y;
-  const int qtile = blockIdx.x / p.dsplit;
-  const int slab = blockIdx.x - qtile * p.dsplit;
+  const int tile = blockIdx.x / p.dsplit;
+  const int slab = blockIdx.x - tile * p.dsplit;
+  // causal: the query tiles run in reverse, heaviest (longest KV extent) first
+  const int qtile = kCausal ? static_cast<int>(gridDim.x) / p.dsplit - 1 - tile : tile;
   const int q0 = qtile * BR;
   const int d0 = slab * p.dv;          // first output column of this CTA
-  const int T = p.num_kv;
+  const int T = kCausal ? attn_kv_tiles(1, p.num_kv, p.Nq, p.Nk, q0 + BR, BC) : p.num_kv;   // KV tiles of this query tile
   const int NVB = p.dv >> 6;           // 64-wide boxes per V chunk
 
   if (warp == 5 && lane == 0) {
@@ -319,6 +324,7 @@ attn_slab_fwd_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_co
     const float c = p.scale_log2;
     float m_run = -INFINITY;
     float l_run = 0.f;
+    const int key_end = kCausal ? attn_key_end(1, p.Nq, p.Nk, q0 + row) : p.Nk;   // keys past it are masked to -inf
 
     for (int j = 0; j < T; ++j) {
       const uint32_t tS = tmem_base + (j & 1) * 128 + lane_field;
@@ -330,7 +336,7 @@ attn_slab_fwd_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_co
       tmem_ld_x32(tS + 64, sreg[2]);
       tmem_ld_x32(tS + 96, sreg[3]);
       tmem_ld_wait();
-      const int valid = p.N - j * BC;
+      const int valid = key_end - j * BC;      // keys of this tile the row sees (the key tail / the diagonal)
       if (valid < BC) {
 #pragma unroll
         for (int cb = 0; cb < 4; ++cb)
@@ -396,8 +402,8 @@ attn_slab_fwd_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_co
     mbar_wait(o_done, (T - 1) & 1, 320);
     tc_fence_after();
     float inv_l = 1.0f / l_run;
-    if (p.lse != nullptr && slab == 0 && (q0 + row) < p.N)
-      p.lse[static_cast<size_t>(bh) * p.N + q0 + row] = 0.6931471805599453f * (m_run * c + log2f(l_run));
+    if (p.lse != nullptr && slab == 0 && (q0 + row) < p.Nq)
+      p.lse[static_cast<size_t>(bh) * p.Nq + q0 + row] = 0.6931471805599453f * (m_run * c + log2f(l_run));
     if (p.rms_g > 0.f) {   // host guarantees dsplit == 1: the whole row is in this thread's lane
       float ss = 0.f;
       for (int cb = 0; cb < (p.dv >> 5); ++cb) {

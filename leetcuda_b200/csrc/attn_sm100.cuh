@@ -29,6 +29,11 @@
 // Shared memory: Q 2 x (128 x DP) fp16, K/V ring of kStages x (128 x DP) fp16, all
 // as 128B-swizzled TMA boxes of 64 columns; the Q buffers are reused to stage O
 // for the TMA store in the epilogue.
+//
+// Nq queries, Nk keys, causal (query row i sees the keys j <= i + Nk - Nq): a work item runs
+// attn_kv_tiles(...) KV tiles, up to the tile holding the last key of its last real row (both
+// query tiles run to tile 1's extent; tile 0 is fully masked on the last one), the per-row key
+// end replaces the ragged-tail mask, and the items are dispatched heaviest first.
 #pragma once
 #include <cuda.h>
 
@@ -55,18 +60,21 @@ struct Cfg {
 };
 
 struct Params {
-  int N;           // sequence length
+  int Nq;          // query rows (q, o, lse)
+  int Nk;          // keys (k, v)
   int D;           // true head dim (<= DP)
-  int num_kv;      // ceil(N / BC)
+  int num_kv;      // ceil(Nk / BC)
+  int causal;      // 1: query row i sees the keys j <= i + Nk - Nq (bottom-right aligned; host guarantees Nk >= Nq)
   float scale_log2;  // softmax scale * log2(e)
   unsigned long long* trace;  // debug: clock64 timeline of CTA (0,0), nullptr = off (B200_FMHA_TRACE)
-  float* lse;      // optional [B*H, N] fp32 output: ln sum_j exp(scale * q.k_j) per query row (the statistic
+  float* lse;      // optional [B*H, Nq] fp32 output: ln sum_j exp(scale * q.k_j) per query row (the statistic
                    // merge_attn_states consumes, cuda_merge_attn_states.cu:19-95); nullptr = off
   float rms_g;     // > 0: RMS-normalise every output row over D in the epilogue (eps 1e-5) and scale by rms_g —
                    // the fused form of kernels/rms-norm/rms_norm.cu:55-110 applied to O; <= 0 = off
   // persistent launches (kPersist): one CTA per SM walks the (batch*head, query-tile-pair) work items
   __half* o_ptr;   // O base pointer: the epilogue stores rows straight from registers (no smem staging)
-  int qpairs;      // ceil(N / 256): work items per (batch, head)
+  int qpairs;      // ceil(Nq / 256): work items per (batch, head)
+  int bhs;         // B * H
   int total_items; // qpairs * B * H
 };
 
@@ -128,7 +136,10 @@ constexpr float kRescaleThreshold = 8.0f;
 //   (3: the classic step on FOUR softmax warpgroups — two threads per query row, warps w and w+4 share 32 TMEM lanes —
 //      was built, verified and measured 5 % slower, profiles/r02_session2l.log, and removed again: the exp loop is bound
 //      by the MUFU pipe of the scheduler both warps sit on, tools/softmax_rate.cu, so a second warp adds nothing.)
-template <int DP, bool kVT, int kStep, bool kPersist>
+//
+// kCausal: the causal mask (Params::causal; the host instantiates it with kStep 0 only).  A separate instantiation keeps
+// the per-row key end, the per-item extent and the reversed order out of the registers of the full-attention kernel.
+template <int DP, bool kVT, int kStep, bool kPersist, bool kCausal>
 __global__ void __launch_bounds__(kThreads, 1)
 attn_fwd_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constant__ CUtensorMap tmap_k,
                 const __grid_constant__ CUtensorMap tmap_v, const __grid_constant__ CUtensorMap tmap_o,
@@ -169,20 +180,29 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constan
   // uniform-datapath descriptor math in the MMA issue loop (no per-instruction R2UR waterfall)
   const int warp = __shfl_sync(0xffffffffu, threadIdx.x >> 5, 0);
   const int lane = threadIdx.x & 31;
-  const int T = p.num_kv;
-  // work items of this CTA: (batch*head, first query row); one-shot launches have exactly one
+  // work items of this CTA: (batch*head, first query row); one-shot launches have exactly one.  Causal work items
+  // are dispatched heaviest first: the one-shot grid runs its query-tile pairs in reverse; the persistent list is
+  // ordered by descending KV extent (all heads of the last query-tile pair, then those of the one before, ...).
   const int w_first = kPersist ? static_cast<int>(blockIdx.x) : 0;
   const int w_step = kPersist ? static_cast<int>(gridDim.x) : 1;
   const int w_total = kPersist ? p.total_items : 1;
   auto item_coords = [&](int w, int& bh, int& q0) {
     if constexpr (kPersist) {
-      bh = w / p.qpairs;
-      q0 = (w - bh * p.qpairs) * (2 * BR);
+      if constexpr (kCausal) {
+        const int r = w / p.bhs;
+        bh = w - r * p.bhs;
+        q0 = (p.qpairs - 1 - r) * (2 * BR);
+      } else {
+        bh = w / p.qpairs;
+        q0 = (w - bh * p.qpairs) * (2 * BR);
+      }
     } else {
       bh = blockIdx.y;
-      q0 = blockIdx.x * (2 * BR);
+      q0 = (kCausal ? static_cast<int>(gridDim.x - 1u - blockIdx.x) : static_cast<int>(blockIdx.x)) * (2 * BR);
     }
   };
+  // KV tiles of the item at q0: both query tiles run to the extent of tile 1 (tile 0 is masked on its last one)
+  auto item_tiles = [&](int q0) { return kCausal ? attn_kv_tiles(1, p.num_kv, p.Nq, p.Nk, q0 + 2 * BR, BC) : p.num_kv; };
 
   if (warp == W_TMA && lane == 0) {
     prefetch_tmap(&tmap_q);
@@ -263,6 +283,7 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constan
       };
       for (int w = w_first; w < w_total; w += w_step, ++it) {
         item_coords(w, bh, q0);
+        const int T = item_tiles(q0);
         load_q(0);
         load_k(0);
         load_q(1);
@@ -310,8 +331,11 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constan
         else if constexpr (kSumSpec) umma_commit(pv_lo_done(t));   // O_t may be rescaled behind this piece
       };
       int it = 0;
+      uint32_t base = 0;   // phases the per-step barriers have completed: the KV extents of the previous items
       for (int w = w_first; w < w_total; w += w_step, ++it) {
-      const uint32_t base = static_cast<uint32_t>(it) * static_cast<uint32_t>(T);   // phases the per-step barriers have completed
+      int bh, q0;
+      item_coords(w, bh, q0);
+      const int T = item_tiles(q0);
       // prologue: S_0(0), S_1(0)
       mbar_wait(q_full(0), it & 1, 200);
       mbar_wait(kv_full(s), ph, 210 + s);
@@ -370,6 +394,7 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constan
         if (more) advance();
         B200_TRACE(2, j, 4);
       }
+      if constexpr (kPersist) base += static_cast<uint32_t>(T);
       }
     }
    }
@@ -384,11 +409,11 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constan
     const uint32_t tO = tmem_o0 + t * DP + lane_field;
     const float c = p.scale_log2;
     const bool tracer = (quarter == 0 && lane == 0);
-    int it = 0;
-    for (int w = w_first; w < w_total; w += w_step, ++it) {
+    uint32_t base = 0;   // phases the per-step barriers have completed: the KV extents of the previous items
+    for (int w = w_first; w < w_total; w += w_step) {
     int bh, q0;
     item_coords(w, bh, q0);
-    const uint32_t base = static_cast<uint32_t>(it) * static_cast<uint32_t>(T);   // phases the per-step barriers have completed
+    const int T = item_tiles(q0);
     float m_run = -INFINITY;  // running (possibly stale) row max of raw S
     float l_run = 0.f;        // running row sum of P
 
@@ -398,7 +423,8 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constan
       mbar_wait(s_full(t), par, 300 + t);
       if (tracer) B200_TRACE(t, j, 1);
       tc_fence_after();
-      const int valid = p.N - j * BC;          // keys of this tile that exist (the tail is masked to -inf)
+      // keys of this tile the row sees (the key tail / the diagonal); the rest is masked to -inf
+      const int valid = (kCausal ? attn_key_end(1, p.Nq, p.Nk, q0 + t * BR + row) : p.Nk) - j * BC;
       // O_t *= alpha in TMEM (lazy rescale; only ever called between two MMAs on O_t, see the callers)
       auto rescale_o = [&](float alpha) {
 #pragma unroll
@@ -418,7 +444,7 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constan
       tmem_ld_x32(tS + 96, sreg[3]);
       tmem_ld_wait();
       if (tracer) B200_TRACE(t, j, 2);
-      // mask the key tail of the last tile
+      // mask the key tail of the last tile and, causal, the keys past the diagonal
       if (valid < BC) {
 #pragma unroll
         for (int cb = 0; cb < 4; ++cb)
@@ -597,11 +623,12 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constan
     // ---------------- epilogue: O / l -> fp16 -> (one-shot) swizzled smem (Q_t buffer) -> TMA store
     //                                             (persistent) straight from registers to global memory
     mbar_wait(o_done(t), (base + static_cast<uint32_t>(T) - 1u) & 1u, 320 + t);
+    if constexpr (kPersist) base += static_cast<uint32_t>(T);
     tc_fence_after();
-    float inv_l = 1.0f / l_run;
     const int qrow = q0 + t * BR + row;
-    if (p.lse != nullptr && qrow < p.N)
-      p.lse[static_cast<size_t>(bh) * p.N + qrow] = 0.6931471805599453f * (m_run * c + log2f(l_run));
+    float inv_l = 1.0f / l_run;
+    if (p.lse != nullptr && qrow < p.Nq)
+      p.lse[static_cast<size_t>(bh) * p.Nq + qrow] = 0.6931471805599453f * (m_run * c + log2f(l_run));
     if (p.rms_g > 0.f) {
       // fused RMS norm: the whole output row of this query sits in this thread's TMEM lane.  One extra
       // pass over the accumulator (TMEM reads are cheap) gives sum(o^2); columns beyond D are exactly 0.
@@ -617,7 +644,7 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constan
       inv_l *= rsqrtf(ss * inv_l * inv_l / static_cast<float>(p.D) + 1e-5f) * p.rms_g;
     }
     if constexpr (kPersist) {
-      __half* orow = p.o_ptr + (static_cast<size_t>(bh) * p.N + qrow) * p.D;
+      __half* orow = p.o_ptr + (static_cast<size_t>(bh) * p.Nq + qrow) * p.D;
 #pragma unroll
       for (int cb = 0; cb < DP / 32; ++cb) {
         uint32_t o[32];
@@ -629,7 +656,7 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constan
           __syncwarp();
           if (lane == 0) mbar_arrive(o_free(t));
         }
-        if (qrow < p.N) {
+        if (qrow < p.Nq) {
 #pragma unroll
           for (int q4 = 0; q4 < 4; ++q4) {
             const int col = cb * 32 + q4 * 8;
@@ -665,7 +692,7 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constan
     }
     fence_proxy_async_smem();
     named_bar_sync(1 + t, 128);
-    if (quarter == 0 && lane == 0 && (q0 + t * BR) < p.N) {
+    if (quarter == 0 && lane == 0 && (q0 + t * BR) < p.Nq) {
 #pragma unroll
       for (int b = 0; b < NBOX; ++b)
         tma_store_3d(&tmap_o, q_base + t * C_::TILE_BYTES + b * C_::BOX_BYTES, b * 64, q0 + t * BR, bh);

@@ -106,4 +106,19 @@ B200_DEVICE float f2_hsum4(const uint64_t (&acc)[4]) {
   return s;
 }
 
+// ---- key extents of causal attention (query row i sees the keys j <= i + Nk - Nq; the host guarantees Nk >= Nq)
+// KV tiles of bc keys a work item with query rows [.., q_end) needs: all num_kv of them, or (causal) those up to the
+// tile holding the last key its last real row sees.  Every role of a kernel derives the item's loop count from this.
+B200_DEVICE int attn_kv_tiles(int causal, int num_kv, int Nq, int Nk, int q_end, int bc) {
+  if (!causal) return num_kv;
+  const int last_key = min(q_end, Nq) - 1 + (Nk - Nq);
+  return min(num_kv, last_key / bc + 1);
+}
+
+// one past the last key query row `qrow` sees: the ragged-tail mask of a tile at key k0 becomes "scores at or beyond
+// key_end - k0 are -inf" (a padding row past Nq keeps a non-empty range; its output is never stored)
+B200_DEVICE int attn_key_end(int causal, int Nq, int Nk, int qrow) {
+  return causal ? min(Nk, qrow + (Nk - Nq) + 1) : Nk;
+}
+
 }  // namespace b200

@@ -15,7 +15,7 @@ from typing import Optional
 
 import torch
 
-from .flash_attn import fmha_fwd
+from .flash_attn import _fmha_ref
 
 __version__ = "0.0.2.b200"
 
@@ -33,12 +33,12 @@ class MMAAccType(Enum):
 
 def ffpa_mma_acc_f32_L1(Q, K, V, O, stages: int = 2) -> None:
     """reference: ffpa-attn/csrc/cuffpa/ffpa_attn_F16F16F32_L1.cu:43-84."""
-    fmha_fwd(Q, K, V, O)
+    _fmha_ref(Q, K, V, O)
 
 
 def ffpa_mma_acc_f16_L1(Q, K, V, O, stages: int = 2) -> None:
     """reference: ffpa-attn/csrc/cuffpa/ffpa_attn_F16F16F16_L1.cu:5-38 (fp32 accumulation here)."""
-    fmha_fwd(Q, K, V, O)
+    _fmha_ref(Q, K, V, O)
 
 
 def faster_prefill_attn_func(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor,

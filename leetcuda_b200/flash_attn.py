@@ -86,22 +86,61 @@ def _check(Q, K, V, O, v_transposed):
     return B, H, N, D
 
 
-def fmha_fwd(Q, K, V, O, *, v_transposed: bool = False, scale: float = 0.0, lse=None) -> None:
+def _check_ex(Q, K, V, O, v_transposed, causal, lse):
+    """Shapes of fmha_fwd: Q, O [B,H,Nq,D]; K [B,H,Nk,D]; V [B,H,Nk,D] or [B,H,D,Nk]; lse fp32 [B,H,Nq]."""
+    for t in (Q, K, V, O):
+        if t.dtype != torch.float16:
+            raise RuntimeError("values must be torch::kHalf")
+    if Q.dim() != 4 or K.dim() != 4:
+        raise RuntimeError("Tensor size mismatch!")
+    B, H, Nq, D = Q.shape
+    Nk = K.shape[2]
+    if tuple(K.shape) != (B, H, Nk, D):
+        raise RuntimeError(f"fmha_fwd: K must be [B,H,Nk,D] = [{B},{H},Nk,{D}], got {list(K.shape)}")
+    if tuple(O.shape) != (B, H, Nq, D):
+        raise RuntimeError(f"fmha_fwd: O must have Q's shape {list(Q.shape)}, got {list(O.shape)}")
+    want_v = (B, H, D, Nk) if v_transposed else (B, H, Nk, D)
+    if tuple(V.shape) != want_v:
+        raise RuntimeError(f"fmha_fwd: V must be {list(want_v)} ({'[B,H,D,Nk]' if v_transposed else '[B,H,Nk,D]'}), "
+                           f"got {list(V.shape)}")
+    if causal and Nk < Nq:
+        raise RuntimeError(f"fmha_fwd: causal attention needs at least as many keys as queries (Nq={Nq}, Nk={Nk}): "
+                           "query row i sees the keys j <= i + Nk - Nq")
+    if lse is not None:
+        if lse.dtype != torch.float32 or tuple(lse.shape) != (B, H, Nq) or not lse.is_cuda or not lse.is_contiguous():
+            raise RuntimeError(f"fmha_fwd: lse must be a contiguous fp32 CUDA tensor [B,H,Nq] = [{B},{H},{Nq}], got "
+                               f"{lse.dtype} {list(lse.shape)}")
+    for t in (Q, K, V, O):
+        if not t.is_cuda:
+            raise RuntimeError("leetcuda_b200.flash_attn: tensors must be CUDA tensors (no CPU path)")
+        if not t.is_contiguous():
+            raise RuntimeError("leetcuda_b200.flash_attn: tensors must be contiguous")
+    return B, H, Nq, Nk, D
+
+
+def fmha_fwd(Q, K, V, O, *, v_transposed: bool = False, scale: float = 0.0, lse=None, causal: bool = False) -> None:
     """``O = softmax(Q K^T * scale) V`` on the current CUDA stream of ``Q``'s device.
 
-    ``lse`` (optional, fp32 ``[B,H,N]`` CUDA tensor) receives ``ln sum_j exp(scale * q_i . k_j)`` per
-    query row — the statistic ``merge_attn_states`` needs to combine results over disjoint key ranges."""
-    B, H, N, D = _check(Q, K, V, O, v_transposed)
+    Q, O: ``[B,H,Nq,D]``; K: ``[B,H,Nk,D]``; V: ``[B,H,Nk,D]`` (``[B,H,D,Nk]`` with ``v_transposed``).
+    ``causal=True``: query row i attends to the keys ``j <= i + Nk - Nq`` (bottom-right alignment, as
+    FlashAttention-2 >= 2.1; top-left, i.e. ``scaled_dot_product_attention(is_causal=True)``, only when Nq == Nk)
+    and needs ``Nk >= Nq``.
+    ``lse`` (optional, fp32 ``[B,H,Nq]`` CUDA tensor) receives ``ln sum_j exp(scale * q_i . k_j)`` over the keys the
+    row attends to — the statistic ``merge_attn_states`` needs to combine results over disjoint key ranges."""
+    B, H, Nq, Nk, D = _check_ex(Q, K, V, O, v_transposed, causal, lse)
     idx = Q.device.index
     args = [Q.data_ptr(), K.data_ptr(), V.data_ptr(), O.data_ptr()]
-    if lse is not None:
-        if lse.dtype != torch.float32 or tuple(lse.shape) != (B, H, N) or not lse.is_cuda or not lse.is_contiguous():
-            raise RuntimeError("leetcuda_b200.flash_attn: lse must be a contiguous fp32 CUDA tensor [B,H,N]")
-        fn = _capi.lib().b200_fmha_fwd_f16_lse
-        args.append(lse.data_ptr())
+    if causal or Nq != Nk:
+        fn = _capi.lib().b200_fmha_fwd_f16_ex
+        args += [None if lse is None else lse.data_ptr(), B, H, Nq, Nk, D, int(v_transposed), int(bool(causal)),
+                 float(scale)]
     else:
-        fn = _capi.lib().b200_fmha_fwd_f16
-    args += [B, H, N, D, int(v_transposed), float(scale)]
+        if lse is not None:
+            fn = _capi.lib().b200_fmha_fwd_f16_lse
+            args.append(lse.data_ptr())
+        else:
+            fn = _capi.lib().b200_fmha_fwd_f16
+        args += [B, H, Nq, D, int(v_transposed), float(scale)]
     if torch.cuda.current_device() != idx:
         with torch.cuda.device(idx):
             rc = fn(*args, _capi.raw_stream(idx))
@@ -133,11 +172,17 @@ def fmha_host(Q, K, V, O, *, v_transposed: bool = False, scale: float = 0.0) -> 
     _capi.check(rc, "fmha_host")
 
 
+def _fmha_ref(Q, K, V, O, v_transposed: bool = False) -> None:
+    """The reference-named ops: equal query / key lengths, full attention, the reference's shape checks."""
+    _check(Q, K, V, O, v_transposed)
+    fmha_fwd(Q, K, V, O, v_transposed=v_transposed)
+
+
 def _make(name: str):
     vt = name in V_TRANSPOSED_OPS
 
     def op(Q, K, V, O, stages: int = 1) -> None:
-        fmha_fwd(Q, K, V, O, v_transposed=vt)
+        _fmha_ref(Q, K, V, O, vt)
     op.__name__ = op.__qualname__ = name
     op.__doc__ = (f"{name}(Q, K, V, O, stages) -> None  "
                   f"[V is {'[B,H,D,N]' if vt else '[B,H,N,D]'}; stages ignored; sm_100a fused kernel]")
@@ -150,7 +195,7 @@ for _n in OP_NAMES:
 
 def flash_attn_cute(Q, K, V, O) -> None:
     """reference: kernels/flash-attn/cutlass/flash_attn_cute.cu:496-524."""
-    fmha_fwd(Q, K, V, O)
+    _fmha_ref(Q, K, V, O)
 
 
 __all__ = OP_NAMES + ["flash_attn_cute", "fmha_fwd", "fmha_host", "OP_NAMES", "V_TRANSPOSED_OPS"]

@@ -58,16 +58,19 @@ def rope_qk(Q, K, Q_out=None, K_out=None) -> None:
     _capi.check(rc, "rope_qk")
 
 
-def attn_rope(Q, K, V, O, *, rms_g: float = 0.0, lse=None) -> None:
+def attn_rope(Q, K, V, O, *, rms_g: float = 0.0, lse=None, causal: bool = False) -> None:
     """``O = attention(rope(Q), rope(K), V)`` (optionally RMS-normalised): the rope pre-pass into scratch copies of
-    Q and K, then the fused attention kernel — two launches."""
+    Q and K, then the fused attention kernel — two launches.  ``causal`` is passed to ``fmha_fwd``; the causal mask
+    with the fused RMS-norm epilogue is not supported."""
+    if causal and rms_g > 0.0:
+        raise RuntimeError("attn_rope: causal attention with the fused RMS-norm epilogue (rms_g > 0) is not supported")
     q_r, k_r = torch.empty_like(Q), torch.empty_like(K)
     rope_qk(Q, K, q_r, k_r)
     if rms_g > 0.0:
         attn_rmsnorm(q_r, k_r, V, O, rms_g, lse=lse)
     else:
         from .flash_attn import fmha_fwd
-        fmha_fwd(q_r, k_r, V, O, lse=lse)
+        fmha_fwd(q_r, k_r, V, O, lse=lse, causal=causal)
 
 
 def bench_rows(torch_mod, dev, steps, peak_hbm, peak_src, cuda_time_ms):
